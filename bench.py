@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — edges/s through the fused gather-message-scatter layer (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 Workload (N=1 default) = BASELINE.json configs[1]: RGCN, synthetic Erdos-Renyi graph, 1M nodes /
 20M edges / 4 edge types, hidden_dim=256, one B200.  A "step" is ONE message-passing layer forward
@@ -56,6 +56,27 @@ WORKLOADS = {
 }
 METRIC = "edges/sec (fused gather-msg-scatter)"
 E2E_DEPTH = int(os.environ.get("TFGNN_B200_E2E_DEPTH", "3"))   # steps in flight in the end-to-end leg (runtime.HostPipeline)
+DUMP_ARRAY_BYTES = 16 << 20   # --dump-outputs, per workload: the three workloads of a default run stay under DUMP_TOTAL_BYTES
+DUMP_TOTAL_BYTES = 64 << 20
+
+
+def dump_rows(V, H):
+    """Rows of a [V, H] float32 layer output that --dump-outputs writes: all of them when they fit DUMP_ARRAY_BYTES, else a
+    fixed seeded sample in ascending order, so that every run (and every build) writes the same rows."""
+    n = DUMP_ARRAY_BYTES // (4 * H)
+    if V <= n:
+        return np.arange(V, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(V, size=n, replace=False))
+
+
+def write_outputs(dirname, outputs):
+    """One DIR/<workload>.npy per measured workload: the sampled rows of its last timed layer call."""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_TOTAL_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_TOTAL_BYTES}-byte limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
 
 
 def algorithmic_bytes(kind, V, E_list, D, H, params):
@@ -505,16 +526,21 @@ def measure_workload(name, args, rank, world, local, dev, headline):
     sampler = ClockSampler(local)
     if headline and rank == 0 and not args.no_clock_sampler:
         sampler.start()          # before the warm-up, so the poller is running when the timed region starts
-    time_device_resident(layer, inp, prepared, 0, args.warmup, None)
-    barrier(world)
-    launches0 = _ffi.launch_count()
-    sampler.begin()
-    total_ms, per_step, out = time_device_resident(layer, inp, prepared, args.steps, 0, flush)
-    sampler.end()
+    try:
+        time_device_resident(layer, inp, prepared, 0, args.warmup, None)
+        barrier(world)
+        launches0 = _ffi.launch_count()
+        sampler.begin()
+        total_ms, per_step, out = time_device_resident(layer, inp, prepared, args.steps, 0, flush)
+        sampler.end()
+    finally:                     # the nvidia-smi poller must not outlive a failed run
+        clocks = sampler.stop() if (headline and rank == 0) else None
     barrier(world)
     launches = _ffi.launch_count() - launches0
     total_ms = max_over_ranks(total_ms, world)
-    clocks = sampler.stop() if (headline and rank == 0) else None
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = out.index_select(0, torch.from_numpy(dump_rows(V, H)).to(dev)).cpu().numpy()
     ms_per_step = total_ms / args.steps
     res = {"workload": wl["desc"], "nodes": V, "edges": M, "edge_types": L, "hidden_dim": H, "kind": kind,
            "ms_per_layer": ms_per_step, "edges_per_s": world * M / (ms_per_step * 1e-3),
@@ -543,7 +569,7 @@ def measure_workload(name, args, rank, world, local, dev, headline):
                                 "frac_of_binding_bound": max(t_hbm_ms, t_dense_ms) / ms_per_step}
     if not args.skip_e2e:
         out_host = torch.empty((V, H), dtype=torch.float32).pin_memory()
-        e2e_steps = max(4, min(args.steps, 10))
+        e2e_steps = args.steps
         dt = time_e2e(layer, h_host, adj_host, out_host, e2e_steps, world, depth=E2E_DEPTH)
         res["e2e"] = {"value": world * M * e2e_steps / dt, "unit": "edges/s",
                       "h2d_bytes_per_step": int(h_host.numel() * 4 + sum(a.numel() * 4 for a in adj_host)),
@@ -553,6 +579,7 @@ def measure_workload(name, args, rank, world, local, dev, headline):
                               f"layer -> D2H(new node states) every step; steps software-pipelined {E2E_DEPTH} deep on CUDA streams "
                               "(runtime.HostPipeline), wall clock over all steps"}
     res["_inputs"] = (h_np, adjs_np, w_np)
+    res["_output"] = dumped
     return res
 
 
@@ -744,6 +771,10 @@ def main():
     ap.add_argument("--skip-secondary", action="store_true", help="headline workload only")
     ap.add_argument("--skip-sharded", action="store_true", help="N > 1: no target-range sharded leg")
     ap.add_argument("--no-clock-sampler", action="store_true", help="do not poll nvidia-smi during the run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write each measured workload's last layer output as DIR/<workload>.npy "
+                         "(float32; all rows, or a fixed seeded sample of 16 MB of rows when larger; rank 0 only) to "
+                         "compare builds on identical seeded inputs")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     wl = WORKLOADS[args.workload]
@@ -764,6 +795,7 @@ def main():
 
     head = measure_workload(args.workload, args, rank, world, local, dev, headline=True)
     h_np, adjs_np, w_np = head.pop("_inputs")
+    outputs = {args.workload: head.pop("_output")}
     V, H, L, M, kind = head["nodes"], head["hidden_dim"], head["edge_types"], head["edges"], head["kind"]
 
     # ---- secondary workloads in the same run (north_star: hidden_dim 320; PPI-shaped batch) ----
@@ -774,6 +806,7 @@ def main():
             r = measure_workload(name, args, rank, world, local, dev, headline=False)
             r.pop("_inputs")
             r.pop("clocks")
+            outputs[name] = r.pop("_output")
             secondary[name] = r
 
     # ---- target-range sharded leg (N > 1) --------------------------------------------------
@@ -784,6 +817,8 @@ def main():
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     cpu = None
     if not args.skip_cpu_baseline and kind == "rgcn":
         threads, _, host_cores = best_cpu_threads(wl, h_np, adjs_np, w_np)

@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -73,6 +74,31 @@ def test_bench_names_a_kernel_per_workload_kind():
     kinds = {w["kind"] for w in bench.WORKLOADS.values()}
     assert kinds <= set(bench.KERNEL_OF)
     assert bench.WORKLOADS["cfg5"]["V"] == 16_000_000 and sum(bench.WORKLOADS["cfg5"]["E"]) > 255_000_000
+
+
+def test_dumped_rows_are_fixed_and_fit_the_limit():
+    """--dump-outputs: the same rows in every run, all rows of a small output, and a default run (cfg2 + h320 + cfg1) within
+    the size limit."""
+    sys.path.insert(0, ROOT)
+    import bench
+    rows = bench.dump_rows(1_000_000, 256)
+    assert np.array_equal(rows, bench.dump_rows(1_000_000, 256))
+    assert np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < 1_000_000
+    assert rows.size * 256 * 4 == bench.DUMP_ARRAY_BYTES
+    assert np.array_equal(bench.dump_rows(8000, 320), np.arange(8000))
+    total = sum(bench.dump_rows(w["V"], w["H"]).size * w["H"] * 4
+                for w in (bench.WORKLOADS[n] for n in ("cfg2", "h320", "cfg1")))
+    assert total <= bench.DUMP_TOTAL_BYTES
+
+
+def test_dump_outputs_refuses_more_than_the_limit(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    with pytest.raises(SystemExit):
+        bench.write_outputs(str(tmp_path / "d"), {"a": np.zeros(bench.DUMP_TOTAL_BYTES // 4 + 1, np.float32)})
+    assert not (tmp_path / "d").exists()
+    bench.write_outputs(str(tmp_path / "d"), {"a": np.ones((3, 2), np.float32)})
+    assert np.array_equal(np.load(tmp_path / "d" / "a.npy"), np.ones((3, 2), np.float32))
 
 
 def test_dropout_stream_offsets_are_disjoint():
